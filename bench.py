@@ -137,6 +137,24 @@ def measured_peak_tensor():
     return 1750.0, "fallback (B200_PROFILING.md dense bf16)"
 
 
+def device_logits(model, vocab: int) -> np.ndarray:
+    """The logits the last forward left on the device (a caller of forward_async reads them from there)."""
+    from ntransformer_b200._lib import lib
+
+    out = np.empty(vocab, np.float32)
+    model.sync()
+    lib().nt_cuda_memcpy_d2h(out.ctypes.data_as(C.c_void_p), C.c_void_p(model.logits_device_ptr), out.nbytes)
+    return out
+
+
+def dump_outputs(out_dir, arrays: dict) -> None:
+    """--dump-outputs: what the timed paths returned in their last step, as DIR/<name>.npy in float32.  The model and the token
+    ids are seeded, so two builds run with the same arguments can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 # ------------------------------------------------------------------------------------------------
 def run_prefill(args, rank, world):
     """BASELINE.json configs[4]: F16 prefill of a whole prompt through the batched tcgen05 path.  One step = one prompt;
@@ -158,7 +176,7 @@ def run_prefill(args, rank, world):
     model = Model.synthetic(cfg, mix, seed=1234)
     stream = torch.cuda.ExternalStream(model.stream)
     vocab = cfg.vocab_size
-    steps = min(args.steps, 16)                                  # a step is a whole prompt
+    steps = args.steps                                           # a step is a whole prompt
     prompts = [[token_at(i + 97 * j, vocab) for i in range(prompt_len)] for j in range(4)]
     for i in range(args.warmup):
         model.forward_async(prompts[i % 4], 0)
@@ -177,12 +195,16 @@ def run_prefill(args, rank, world):
     launches = K.launch_count() - launches0
     clocks = sampler.stop()
     tok_s = steps * prompt_len / (ms / 1e3)
+    outputs = {"logits": device_logits(model, vocab)} if args.dump_outputs else None
     # end to end
     t0 = time.perf_counter()
     for i in range(steps):
         logits = model.forward(prompts[i % 4], 0)
     e2e_ms = (time.perf_counter() - t0) * 1e3
     assert np.isfinite(logits).all(), "non-finite logits"
+    if outputs is not None:
+        outputs["e2e_logits"] = logits.copy()
+        dump_outputs(args.dump_outputs, outputs)
     # per-token replay of the decode step (what the reference's forward loop does, on our kernels) for comparison
     model.set_prefill_min_tokens(0)
     n_cmp = min(prompt_len, 64)
@@ -272,7 +294,7 @@ def run_ours(args, rank, world):
     torch.cuda.set_device(local)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-    line = measure_decode(args, rank, world, args.workload, with_cpu=not args.no_cpu_baseline)
+    line = measure_decode(args, rank, world, args.workload, with_cpu=not args.no_cpu_baseline, dump_dir=args.dump_outputs)
     # BASELINE.json configs[3] (70B Q6_K, 8-way tensor parallel) rides along with the 8-GPU run of the metric's own config
     # (Q4_K_M at every N, so that the 1/2/4/8 series stays one workload): reported under "configs3".
     if world == 8 and args.workload == "llama3-70b-q4_k_m-decode" and not args.no_configs3:
@@ -286,7 +308,7 @@ def run_ours(args, rank, world):
         dist.destroy_process_group()
 
 
-def measure_decode(args, rank, world, workload, with_cpu):
+def measure_decode(args, rank, world, workload, with_cpu, dump_dir=None):
     import torch
     import torch.distributed as dist
     from ntransformer_b200 import kernels as K
@@ -337,6 +359,7 @@ def measure_decode(args, rank, world, workload, with_cpu):
     ms = ev0.elapsed_time(ev1)
     launches = K.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    outputs = {"logits": device_logits(model, vocab)} if dump_dir and rank == 0 else None
     if world > 1:
         t = torch.tensor([ms], device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -366,6 +389,9 @@ def measure_decode(args, rank, world, workload, with_cpu):
         e2e_ms = float(t.item())
     e2e_tok_s = args.steps / (e2e_ms / 1e3)
     assert np.isfinite(logits).all(), "non-finite logits"
+    if outputs is not None:
+        outputs["e2e_logits"] = logits.copy()
+        dump_outputs(dump_dir, outputs)
     tp_info = None
     if world > 1:
         # tensor-parallel lock-step: every rank must hold bit-identical logits (the replicas sample the same token)
@@ -563,7 +589,7 @@ def run_reference(args, rank, world):
             # so its prompt rate does not depend on the prompt length apart from the attention term: a 128-token prompt per
             # step is the bounded sample of the 4096-token workload.
             n_ref = min(prompt_len, 128)
-            steps = min(args.steps, 4)
+            steps = args.steps
             logits = np.empty(vocab, np.float32)
             toks = np.array([token_at(i, vocab) for i in range(n_ref)], np.int32)
             ref.ref_model_forward(h, toks.ctypes.data_as(C.c_void_p), min(n_ref, 8), 0, None)          # warm-up
@@ -577,6 +603,8 @@ def run_reference(args, rank, world):
             ms = (time.perf_counter() - t0) * 1e3
             clocks = sampler.stop()
             ref.ref_model_free(h)
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, {"logits": logits})
             tok_s = steps * n_ref / (ms / 1e3)
             print(json.dumps({
                 "impl": "reference", "metric": "prefill_tok_s", "value": round(tok_s, 2), "unit": "tok/s", "n_gpus": 1, "steps": steps,
@@ -614,6 +642,8 @@ def run_reference(args, rank, world):
         ms = (time.perf_counter() - t0) * 1e3
         clocks = sampler.stop()
         ref.ref_model_free(h)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"logits": logits})
     finally:
         if os.path.exists(path):
             os.unlink(path)
@@ -638,11 +668,19 @@ def run_check(args, rank, world):
     """Parity at the benchmarked configuration (not a timing): the workload's seeded model is written to a GGUF once, loaded by
     the reference (oracle/_ref: its own loader + CUDA kernels, sm_100 build) and by our engine, and both decode greedily from the
     same prompt.  Asserts logits <= 1e-3 relative (max |a - b| / max |b|) at every step where the histories agree and identical
-    greedy ids for --steps tokens.  One GPU (the reference is single-GPU); prints one JSON line."""
+    greedy ids for --steps tokens.  One GPU (the reference is single-GPU); prints one JSON line.
+
+    With --reference-trace the reference's side is read from a recording (oracle/trace.py) instead of oracle/_ref, so the
+    check runs without the reference; --record-reference-trace writes that recording from a live run."""
     if rank != 0:
         return
+    from oracle.trace import Recorder, Trace
+
     so = ROOT / "oracle" / "_ref" / "libnt_ref.so"
-    if not so.exists():
+    replay = None
+    if args.reference_trace:
+        replay = np.load(args.reference_trace)
+    elif not so.exists():
         print(json.dumps({"check": args.workload, "unavailable": "oracle/_ref/libnt_ref.so was not built"}))
         return
     import torch
@@ -656,6 +694,13 @@ def run_check(args, rank, world):
     if args.layers:                                   # a slice of the stack with full-width tensors (70B shapes in seconds)
         from dataclasses import replace
         cfg = replace(cfg, n_layers=args.layers)
+    p_len = min(prompt_len, 16)                       # the reference prefills token by token
+    meta = {"workload": args.workload, "layers": cfg.n_layers, "steps": args.steps, "prompt_tokens": p_len,
+            "oracle_steps": args.oracle_steps}
+    if replay is not None:
+        recorded = json.loads(str(replay["meta"]))
+        assert recorded == meta, f"{args.reference_trace} records {recorded}, not {meta}"
+        trace = Trace(replay)
     torch.cuda.set_device(0)
     tmpdir = "/dev/shm" if os.path.isdir("/dev/shm") else tempfile.gettempdir()
     path = os.path.join(tmpdir, f"nt_check_{args.workload}_{os.getpid()}.gguf")
@@ -672,31 +717,43 @@ def run_check(args, rank, world):
             yield name, t.cpu().numpy(), dt, rows, cols
     write_gguf_streaming(path, cfg, gen(), tensor_table(cfg, mix))
     try:
-        ref = C.CDLL(str(so))
-        ref.ref_model_load.restype = C.c_void_p
-        ref.ref_model_load.argtypes = [C.c_char_p, C.c_int]
-        ref.ref_model_forward.restype = C.c_float
-        ref.ref_model_forward.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]
-        ref.ref_model_free.argtypes = [C.c_void_p]
+        ref = h = None
         devnull, saved = os.open(os.devnull, os.O_WRONLY), os.dup(2)
         os.dup2(devnull, 2)
         try:
-            h = ref.ref_model_load(path.encode(), max_seq)
+            if replay is None:
+                ref = C.CDLL(str(so))
+                ref.ref_model_load.restype = C.c_void_p
+                ref.ref_model_load.argtypes = [C.c_char_p, C.c_int]
+                ref.ref_model_forward.restype = C.c_float
+                ref.ref_model_forward.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]
+                ref.ref_model_free.argtypes = [C.c_void_p]
+                h = ref.ref_model_load(path.encode(), max_seq)
             ours = Model.load(path, max_seq)
         finally:
             os.dup2(saved, 2)
             os.close(devnull)
-        assert h, "reference failed to load the GGUF"
+        assert replay is not None or h, "reference failed to load the GGUF"
         vocab = cfg.vocab_size
-        p_len = min(prompt_len, 16)                    # the reference prefills token by token
         toks = np.array([token_at(i, vocab) for i in range(p_len)], np.int32)
         lr = np.empty(vocab, np.float32)
-        ref.ref_model_forward(h, toks.ctypes.data_as(C.c_void_p), p_len, 0, lr.ctypes.data_as(C.c_void_p))
+        rec = Recorder(vocab) if args.record_reference_trace else None
+        rel = lambda a, b: float(np.abs(a - b).max() / np.abs(b).max())
+
+        def ref_step(step, t, n, pos, lo):
+            """The reference's greedy id after this forward and the relative error of our logits lo against its logits."""
+            if replay is not None:
+                return trace.greedy(step), trace.rel_err(step, lo)
+            ref.ref_model_forward(h, t.ctypes.data_as(C.c_void_p), n, pos, lr.ctypes.data_as(C.c_void_p))
+            if rec:
+                rec.add(lr)
+            return int(np.argmax(lr)), rel(lo, lr)
+
         if args.per_token_prompt:
             ours.set_prefill_min_tokens(0)
         lo = ours.forward([int(t) for t in toks], 0).copy()          # 16 tokens: the batched tensor-core prefill, as a user gets it
-        rel = lambda a, b: float(np.abs(a - b).max() / np.abs(b).max())
-        errs = [rel(lo, lr)]
+        tr, err = ref_step(0, toks, p_len, 0, lo)
+        errs = [err]
         # conditioning of the synthetic model: the F64-accumulating CPU oracle on the same weights tells how far two correct F32
         # implementations may drift apart (random weights make a deep stack chaotic; a trained checkpoint is far better behaved)
         cond = None
@@ -707,25 +764,30 @@ def run_check(args, rank, world):
             c["max_seq_len"] = p_len + args.oracle_steps + 4
             om = O.Model(c, host)
             lq = om.forward([int(t) for t in toks], 0)
-            cond = {"ref_vs_f64": [rel(lr, lq)], "ours_vs_f64": [rel(lo, lq)]}
-        ids_o, ids_r, to, tr, pos, agree, first_bad = [], [], int(np.argmax(lo)), int(np.argmax(lr)), p_len, True, None
+            cond = {"ref_vs_f64": [None if replay is not None else rel(lr, lq)], "ours_vs_f64": [rel(lo, lq)]}
+        ids_o, ids_r, to, pos, agree, first_bad = [], [], int(np.argmax(lo)), p_len, True, None
         for step in range(args.steps):
             ids_o.append(to)
             ids_r.append(tr)
-            t = np.array([tr], np.int32)
-            ref.ref_model_forward(h, t.ctypes.data_as(C.c_void_p), 1, pos, lr.ctypes.data_as(C.c_void_p))
             lo = ours.forward([to], pos).copy()
+            tr_next, err = ref_step(step + 1, np.array([tr], np.int32), 1, pos, lo)
             if agree and to != tr:
                 agree, first_bad = False, step
             if agree:
-                errs.append(rel(lo, lr))
+                errs.append(err)
                 if cond is not None and step < args.oracle_steps:
                     lq = om.forward([tr], pos)
-                    cond["ref_vs_f64"].append(rel(lr, lq))
+                    cond["ref_vs_f64"].append(None if replay is not None else rel(lr, lq))
                     cond["ours_vs_f64"].append(rel(lo, lq))
-            to, tr, pos = int(np.argmax(lo)), int(np.argmax(lr)), pos + 1
+            to, tr, pos = int(np.argmax(lo)), tr_next, pos + 1
         worst = max(errs)
-        ref.ref_model_free(h)
+        if cond is not None and replay is not None:
+            cond["ref_vs_f64"] = [float(v) for v in replay["ref_vs_f64"][:len(cond["ours_vs_f64"])]]
+        if rec:
+            np.savez_compressed(args.record_reference_trace, meta=json.dumps(meta), **rec.arrays(),
+                                ref_vs_f64=np.array(cond["ref_vs_f64"] if cond else [], np.float64))
+        if h:
+            ref.ref_model_free(h)
         ours.close()
     finally:
         if os.path.exists(path):
@@ -734,16 +796,24 @@ def run_check(args, rank, world):
     # distance from the F64 result within twice the reference's own (+1e-4): deep stacks of random blocks are ill-conditioned, the
     # reference's F32 path itself drifts up to 2.9e-3 from exact arithmetic on an 8-layer 8B slice over 128 steps (profiles/r02_parity_8b.txt).
     ok = ids_o == ids_r and worst <= 1e-3
-    if not ok and ids_o == ids_r and cond is not None:
+    f64_ok = None
+    if cond is not None:
         r_err, o_err = max(cond["ref_vs_f64"]), max(cond["ours_vs_f64"])
-        ok = o_err <= 2.0 * r_err + 1e-4 and worst <= 2.0 * r_err + 1e-3
+        f64_ok = o_err <= 2.0 * r_err + 1e-4
+    if not ok and ids_o == ids_r and f64_ok is not None:
+        ok = f64_ok and worst <= 2.0 * r_err + 1e-3
+    # A recording keeps the reference's logits at a few positions only (oracle/trace.py), so there the full-vocabulary distance
+    # from the F64 result must hold as well.
+    if replay is not None and f64_ok is not None:
+        ok = ok and f64_ok
     if cond is not None:
         cond = {k: [float("%.3g" % v) for v in vs] for k, vs in cond.items()}
+    against = ("a recording of oracle/_ref (%s)" % Path(args.reference_trace).name if replay is not None else
+               "oracle/_ref (the reference's loader + CUDA kernels + Transformer::forward, sm_100 build), same GGUF")
     print(json.dumps({"check": args.workload, "layers": cfg.n_layers, "steps": args.steps, "prompt_tokens": p_len,
                       "max_rel_logit_err": worst, "err_after_prompt": errs[0], "err_first_steps": [float("%.3g" % e) for e in (errs[1:] if args.all_errs else errs[1:9])],
                       "first_id_mismatch_step": first_bad, "conditioning": cond,
-                      "tolerance": 1e-3, "greedy_ids_identical": ids_o == ids_r, "ok": ok,
-                      "against": "oracle/_ref (the reference's loader + CUDA kernels + Transformer::forward, sm_100 build), same GGUF"}),
+                      "tolerance": 1e-3, "greedy_ids_identical": ids_o == ids_r, "ok": ok, "against": against}),
           flush=True)
     if not ok:
         sys.exit(1)
@@ -752,7 +822,9 @@ def run_check(args, rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=128)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default: 128 decoded tokens; for prefill workloads, where a step is a whole prompt, 16, "
+                         "and 4 with --impl reference)")
     ap.add_argument("--warmup", type=int, default=8)
     ap.add_argument("--workload", default="llama3-70b-q4_k_m-decode", choices=sorted(WORKLOADS))
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
@@ -766,7 +838,17 @@ def main():
     ap.add_argument("--oracle-steps", type=int, default=0, help="--check only: also run the F64-accumulating CPU oracle for the prompt and this many steps")
     ap.add_argument("--all-errs", action="store_true", help="--check only: list the error of every step, not the first 8")
     ap.add_argument("--per-token-prompt", action="store_true", help="--check only: our engine replays the prompt token by token like the reference")
+    ap.add_argument("--reference-trace", default=None,
+                    help="--check only: compare with this recording of the reference (oracle/trace.py .npz) instead of oracle/_ref")
+    ap.add_argument("--record-reference-trace", default=None, help="--check only: write the reference's side of the check to this .npz")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write the logits of the last timed step of each timed path to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps is None:
+        prefill = "prefill" in args.workload and not args.check
+        args.steps = (4 if args.impl == "reference" else 16) if prefill else 128
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))

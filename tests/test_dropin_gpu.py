@@ -32,7 +32,7 @@ def _bind(lib):
 def dropin_lib():
     p = ROOT / "oracle" / "_ref" / "libnt_dropin.so"
     if not p.exists():
-        pytest.skip("oracle/_ref/libnt_dropin.so not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libnt_dropin.so not built (build() with NT_REFERENCE_SRC set compiles it)")
     return _bind(C.CDLL(str(p)))
 
 

@@ -1,9 +1,12 @@
 """GPU parity tests: every entry point is called through the C-ABI of libnt_b200.so and compared with the CPU
-oracle on the same seeded inputs; where oracle/_ref travelled, also with the reference's own CUDA kernels.
+oracle on the same seeded inputs, and with what the reference's own CUDA kernels computed from those inputs
+(tests/golden/ref_kernels.npz, recorded by tests/golden/make_ref_golden.py).
 
 Tolerances (floating point, stated per test): GEMV max|d| <= 2e-5 * max|y| against the F64-accumulating
 oracle (BASELINE north_star allows 1e-3 on logits); attention 2e-5 abs on O(1) outputs."""
 import ctypes as C
+import hashlib
+from pathlib import Path
 
 import numpy as np
 import pytest
@@ -16,6 +19,13 @@ from oracle import oracle as O
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
+GOLDEN = Path(__file__).resolve().parent / "golden" / "ref_kernels.npz"
+
+
+@pytest.fixture(scope="module")
+def golden():
+    with np.load(GOLDEN) as g:
+        return dict(g)
 
 
 def dev(a):
@@ -50,23 +60,30 @@ def test_gemv_vs_oracle(dt, shape):
     assert rel_err(y.cpu().numpy(), ref) <= 2e-5
 
 
-@pytest.mark.parametrize("dt", [DType.Q4_K_M, DType.Q5_K, DType.Q6_K, DType.Q8_0, DType.Q4_0, DType.F16])
-@pytest.mark.parametrize("shape", [(64, 4096), (40, 8192), (12, 28672)])
-def test_gemv_vs_reference_cuda(ref_lib, dt, shape):
+REF_GEMV_DT = [DType.Q4_K_M, DType.Q5_K, DType.Q6_K, DType.Q8_0, DType.Q4_0, DType.F16]
+REF_GEMV_SHAPES = [(64, 4096), (40, 8192), (12, 28672)]
+
+
+def ref_gemv_case(dt, shape):
+    """Inputs of test_gemv_vs_reference_cuda and the key of the reference's output in the golden file."""
     out, inn = shape
-    if dt in (DType.Q8_0, DType.Q4_0, DType.F16) and inn * 4 > 64 * 1024:
-        pytest.skip("reference kernel needs > 64 KB dynamic smem for this dtype (SURVEY 3.3) and fails to launch")
     rng = np.random.default_rng(out + inn + 17 * int(dt))
     raw = random_blocks_np(dt, out, inn, rng)
     x = rng.standard_normal(inn).astype(np.float32)
-    W, xd = dev(raw), dev(x)
+    return raw, x, f"gemv_{dt.name}_{out}x{inn}"
+
+
+@pytest.mark.parametrize("dt", REF_GEMV_DT)
+@pytest.mark.parametrize("shape", REF_GEMV_SHAPES)
+def test_gemv_vs_reference_cuda(golden, dt, shape):
+    out, inn = shape
+    if dt in (DType.Q8_0, DType.Q4_0, DType.F16) and inn * 4 > 64 * 1024:
+        pytest.skip("reference kernel needs > 64 KB dynamic smem for this dtype (SURVEY 3.3) and fails to launch")
+    raw, x, key = ref_gemv_case(dt, shape)
     y = torch.zeros(out, device=DEV)
-    yr = torch.zeros(out, device=DEV)
-    K.launch_gemv(y, W, xd, out, inn, dt)
-    s = torch.cuda.current_stream().cuda_stream
-    ref_lib.ref_gemv(C.c_void_p(yr.data_ptr()), C.c_void_p(W.data_ptr()), C.c_void_p(xd.data_ptr()), out, inn, int(dt), C.c_void_p(s))
+    K.launch_gemv(y, dev(raw), dev(x), out, inn, dt)
     sync()
-    assert rel_err(y.cpu().numpy(), yr.cpu().numpy()) <= 2e-5
+    assert rel_err(y.cpu().numpy(), golden[key]) <= 2e-5
 
 
 def f16bits(v):
@@ -207,19 +224,32 @@ def test_rope_and_kv_cache(interleaved, request):
     np.testing.assert_array_equal(vc.cpu().numpy().view(np.uint16), vcw)
 
 
-def test_rope_matches_reference_cuda_bitwise(ref_lib):
+ROPE_SHAPE = (7, 64, 8, 128)                                     # seq, n_heads, n_kv_heads, head_dim
+
+
+def ref_rope_case():
     rng = np.random.default_rng(80)
-    seq, nh, nkv, hd = 7, 64, 8, 128
+    seq, nh, nkv, hd = ROPE_SHAPE
     q = rng.standard_normal((seq, nh, hd)).astype(np.float32)
     k = rng.standard_normal((seq, nkv, hd)).astype(np.float32)
-    pos = dev(np.array([0, 1, 100, 1000, 2047, 4095, 8191], np.int32))
-    qa, ka, qb, kb = dev(q), dev(k), dev(q), dev(k)
-    K.launch_rope(qa, ka, pos, 1, seq, nh, nkv, hd, 500000.0, 1.0, False)
-    s = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-    ref_lib.ref_rope(C.c_void_p(qb.data_ptr()), C.c_void_p(kb.data_ptr()), C.c_void_p(pos.data_ptr()), 1, seq, nh, nkv, hd,
-                     C.c_float(500000.0), C.c_float(1.0), 0, s)
+    return q, k, np.array([0, 1, 100, 1000, 2047, 4095, 8191], np.int32)
+
+
+def sha256(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def test_rope_matches_reference_cuda_bitwise(golden):
+    """The golden file keeps the SHA-256 of the reference's rotated q and k (bit-exact comparison) and every 16th value."""
+    seq, nh, nkv, hd = ROPE_SHAPE
+    q, k, pos = ref_rope_case()
+    qa, ka = dev(q), dev(k)
+    K.launch_rope(qa, ka, dev(pos), 1, seq, nh, nkv, hd, 500000.0, 1.0, False)
     sync()
-    assert torch.equal(qa, qb) and torch.equal(ka, kb)           # same fast-math instruction sequence
+    qo, ko = qa.cpu().numpy(), ka.cpu().numpy()
+    np.testing.assert_array_equal(qo.reshape(-1)[::16], golden["rope_q_every16"])
+    np.testing.assert_array_equal(ko.reshape(-1)[::16], golden["rope_k_every16"])
+    assert (sha256(qo), sha256(ko)) == (str(golden["rope_q_sha256"]), str(golden["rope_k_sha256"]))   # same fast-math instruction sequence
 
 
 def test_elementwise_ops():
@@ -294,23 +324,29 @@ def test_attention_decode_vs_oracle(cfg, ctx):
     np.testing.assert_allclose(out.cpu().numpy(), want, atol=2e-5, rtol=1e-4)
 
 
-@pytest.mark.parametrize("cfg", [(32, 8, 128), (64, 8, 128)])
-@pytest.mark.parametrize("ctx", [17, 2048])
-def test_attention_decode_vs_reference_cuda(ref_lib, cfg, ctx):
+REF_ATTN_CFGS, REF_ATTN_CTX = [(32, 8, 128), (64, 8, 128)], [17, 2048]
+
+
+def ref_attention_case(cfg, ctx):
+    """Inputs of test_attention_decode_vs_reference_cuda and the key of the reference's output in the golden file."""
     nh, nkv, hd = cfg
     rng = np.random.default_rng(nh + ctx)
-    max_seq = 2048
-    kc, vc = make_cache(rng, max_seq, nkv, hd)
+    kc, vc = make_cache(rng, 2048, nkv, hd)
     q = rng.standard_normal((nh, hd)).astype(np.float32)
+    return q, kc, vc, f"attn_{nh}_{nkv}_{hd}_ctx{ctx}"
+
+
+@pytest.mark.parametrize("cfg", REF_ATTN_CFGS)
+@pytest.mark.parametrize("ctx", REF_ATTN_CTX)
+def test_attention_decode_vs_reference_cuda(golden, cfg, ctx):
+    nh, nkv, hd = cfg
+    max_seq = 2048
+    q, kc, vc, key = ref_attention_case(cfg, ctx)
     scale = float(1.0 / np.sqrt(hd))
-    a, b = torch.zeros(nh, hd, device=DEV), torch.zeros(nh, hd, device=DEV)
-    qd, kd, vd = dev(q), dev(kc), dev(vc)
-    K.launch_attention_decode(a, qd, kd, vd, ctx, nh, nkv, hd, max_seq, scale)
-    s = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-    ref_lib.ref_attention_decode(C.c_void_p(b.data_ptr()), C.c_void_p(qd.data_ptr()), C.c_void_p(kd.data_ptr()),
-                                 C.c_void_p(vd.data_ptr()), ctx, nh, nkv, hd, max_seq, C.c_float(scale), s)
+    a = torch.zeros(nh, hd, device=DEV)
+    K.launch_attention_decode(a, dev(q), dev(kc), dev(vc), ctx, nh, nkv, hd, max_seq, scale)
     sync()
-    np.testing.assert_allclose(a.cpu().numpy(), b.cpu().numpy(), atol=2e-5, rtol=1e-4)
+    np.testing.assert_allclose(a.cpu().numpy(), golden[key], atol=2e-5, rtol=1e-4)
 
 
 @pytest.mark.parametrize("cfg", [(32, 8, 128), (4, 2, 64)])

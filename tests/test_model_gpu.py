@@ -1,8 +1,8 @@
 """GPU model-level parity: the native engine (CUDA graph, fused launches) against the CPU oracle on the same
-synthetic weights, against the reference's own Transformer::forward (oracle/_ref) on the same GGUF file, and
-through the reference's declared C API (include/ntransformer.h).  Tolerance: max|logit diff| / max|logit|
-<= 1e-3 (BASELINE.json north_star) — measured values are ~1e-5 — and greedy token ids identical."""
-import ctypes as C
+synthetic weights, against the reference's own Transformer::forward on the same GGUF file (its greedy decode
+recorded under tests/golden/ by tests/golden/make_ref_golden.py, see oracle/trace.py), and through the reference's
+declared C API (include/ntransformer.h).  Tolerance: max|logit diff| / max|logit| <= 1e-3 (BASELINE.json
+north_star) — measured values are ~1e-5 — and greedy token ids identical."""
 import subprocess
 import sys
 from pathlib import Path
@@ -16,9 +16,11 @@ from ntransformer_b200.engine import Engine, Model
 from ntransformer_b200.gguf_write import synthetic_tensors_np, write_gguf
 from ntransformer_b200.model_spec import TINY, LlamaConfig
 from oracle import oracle as O
+from oracle.trace import Trace
 
 pytestmark = pytest.mark.gpu
 ROOT = Path(__file__).resolve().parent.parent
+GOLDEN = ROOT / "tests" / "golden"
 
 MID = LlamaConfig(vocab_size=2048, hidden_size=1024, intermediate_size=3584, n_layers=4, n_heads=16, n_kv_heads=4, head_dim=64,
                   max_seq_len=256, bos_token_id=1, eos_token_id=2)
@@ -28,13 +30,18 @@ def rel(a, b):
     return float(np.abs(a - b).max() / np.abs(b).max())
 
 
+def write_case(mix, d):
+    cfg = TINY if mix != "Q6_K" else MID
+    tensors = synthetic_tensors_np(cfg, mix, seed=11)
+    path = d / f"{mix}.gguf"
+    write_gguf(path, cfg, tensors)
+    return cfg, tensors, path
+
+
 @pytest.fixture(scope="module", params=["Q4_K_M", "Q8_0", "Q6_K", "F16"])
 def gguf_case(request, tmp_path_factory):
     mix = request.param
-    cfg = TINY if mix != "Q6_K" else MID
-    tensors = synthetic_tensors_np(cfg, mix, seed=11)
-    path = tmp_path_factory.mktemp("m") / f"{mix}.gguf"
-    write_gguf(path, cfg, tensors)
+    cfg, tensors, path = write_case(mix, tmp_path_factory.mktemp("m"))
     host = {n: (np.ascontiguousarray(a), int(dt)) for n, (a, dt, r, c) in tensors.items()}
     return cfg, mix, path, host
 
@@ -107,32 +114,28 @@ def test_batched_tensor_core_prefill_vs_oracle_and_per_token(tmp_path, mix, n_pr
     a.close(), b.close()
 
 
-def test_vs_reference_transformer_forward(ref_lib, gguf_case):
+REF_PROMPT, REF_STEPS = [1, 17, 300, 5, 44, 9], 32
+
+
+def test_vs_reference_transformer_forward(gguf_case):
+    """The reference's greedy decode of the same GGUF, recorded: its ids and, per step, its logits at the positions oracle/trace.py
+    keeps (the largest ones and a fixed sample)."""
     cfg, mix, path, host = gguf_case
-    ref_lib.ref_model_load.restype = C.c_void_p
-    ref_lib.ref_model_load.argtypes = [C.c_char_p, C.c_int]
-    ref_lib.ref_model_forward.restype = C.c_float
-    ref_lib.ref_model_forward.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]
-    ref_lib.ref_model_free.argtypes = [C.c_void_p]
-    h = ref_lib.ref_model_load(str(path).encode(), cfg.max_seq_len)
-    assert h
+    with np.load(GOLDEN / f"ref_forward_{mix}.npz") as g:
+        ref = Trace(g)
+    assert len(ref) == REF_STEPS + 1
     m = Model.load(path, cfg.max_seq_len)
-    prompt = np.array([cfg.bos_token_id, 17, 300, 5, 44, 9], np.int32)
-    ref_logits = np.empty(cfg.vocab_size, np.float32)
-    ref_lib.ref_model_forward(h, prompt.ctypes.data_as(C.c_void_p), len(prompt), 0, ref_logits.ctypes.data_as(C.c_void_p))
+    prompt = np.array(REF_PROMPT, np.int32)
     ours = m.forward(prompt, 0).copy()
-    assert rel(ours, ref_logits) <= 1e-3
-    pos, ta, tb, ida, idb = len(prompt), int(np.argmax(ours)), int(np.argmax(ref_logits)), [], []
-    for _ in range(32):
+    assert ref.rel_err(0, ours) <= 1e-3
+    pos, ta, tb, ida, idb = len(prompt), int(np.argmax(ours)), ref.greedy(0), [], []
+    for step in range(1, REF_STEPS + 1):
         ida.append(ta)
         idb.append(tb)
-        t = np.array([tb], np.int32)
-        ref_lib.ref_model_forward(h, t.ctypes.data_as(C.c_void_p), 1, pos, ref_logits.ctypes.data_as(C.c_void_p))
         la = m.forward([ta], pos).copy()
-        assert ta != tb or rel(la, ref_logits) <= 1e-3
-        ta, tb, pos = int(np.argmax(la)), int(np.argmax(ref_logits)), pos + 1
+        assert ta != tb or ref.rel_err(step, la) <= 1e-3
+        ta, tb, pos = int(np.argmax(la)), ref.greedy(step), pos + 1
     assert ida == idb                                        # greedy ids bit-exact with the reference CUDA path
-    ref_lib.ref_model_free(h)
     m.close()
 
 
@@ -163,18 +166,27 @@ def test_c_api_engine_and_cli(gguf_case):
     assert r2.returncode == 1 and "not supported" in r2.stderr
 
 
-@pytest.mark.parametrize("workload,layers,steps,extra", [
+PARITY_CONFIGS = [
     ("llama3-8b-q4_k_m-decode", 8, 64, ["--oracle-steps", "64"]), ("llama3-8b-q8_0-decode", 8, 64, ["--oracle-steps", "64"]),
     ("llama3-70b-q4_k_m-decode", 4, 48, ["--oracle-steps", "48"]), ("llama3-70b-q6_k-decode", 4, 48, ["--oracle-steps", "48"]),
-    ("llama3-8b-q4_k_m-decode", 0, 24, ["--oracle-steps", "3"])])
-def test_parity_at_the_benchmarked_configs(ref_lib, workload, layers, steps, extra):
+    ("llama3-8b-q4_k_m-decode", 0, 24, ["--oracle-steps", "3"])]
+
+
+def parity_trace(workload, layers):
+    return GOLDEN / f"ref_check_{workload}_{layers}l.npz"
+
+
+@pytest.mark.parametrize("workload,layers,steps,extra", PARITY_CONFIGS)
+def test_parity_at_the_benchmarked_configs(workload, layers, steps, extra):
     """bench.py --check: the benchmark's own seeded weights (8-layer slices of the 8B shapes, 4-layer slices of the 70B shapes with
-    full-width tensors, and the full 32-layer 8B stack) through the reference's CUDA path and ours from the same GGUF, the F64 oracle
-    beside them.  Greedy ids must be identical; logits within 1e-3 of the reference, or — these stacks of random blocks are
-    ill-conditioned: the reference's own F32 path drifts up to 2.9e-3 from the F64 result over 128 steps on the 8-layer slice, ours
-    2.8e-3 (profiles/r02_parity_8b.txt) — our distance from the F64 result within twice the reference's (bench.py run_check)."""
+    full-width tensors, and the full 32-layer 8B stack) through ours, against the reference's CUDA path on the same GGUF (recorded
+    by tests/golden/make_ref_golden.py: bench.py --check --record-reference-trace), the F64 oracle beside them.  Greedy ids must be
+    identical; logits within 1e-3 of the reference, or — these stacks of random blocks are ill-conditioned: the reference's own F32
+    path drifts up to 2.9e-3 from the F64 result over 128 steps on the 8-layer slice, ours 2.8e-3 (profiles/r02_parity_8b.txt) — our
+    distance from the F64 result within twice the reference's (bench.py run_check)."""
     import json
-    cmd = [sys.executable, str(ROOT / "bench.py"), "--check", "--workload", workload, "--steps", str(steps)] + extra
+    cmd = [sys.executable, str(ROOT / "bench.py"), "--check", "--workload", workload, "--steps", str(steps),
+           "--reference-trace", str(parity_trace(workload, layers))] + extra
     if layers:
         cmd += ["--layers", str(layers)]
     r = subprocess.run(cmd, capture_output=True, text=True, timeout=1500)

@@ -1,10 +1,11 @@
-"""Host-side parity against the UNMODIFIED reference code (oracle/_ref/libnt_ref.so, built from /root/reference by
-oracle/Makefile; skipped when it was not built): our GGUF parser, tokenizer and sampler (csrc/engine/{gguf,text}.cpp) against
-the reference's GGUFLoader (src/model/loader.cpp:23-276), Tokenizer (src/inference/tokenizer.cpp:64-314) and Sampler
-(src/inference/sampler.cpp:18-117) on the same files and inputs.  No GPU is involved: these are the host rows (a17, a18) of
-SURVEY §8, which the reference's own tests do not pin."""
+"""Host-side parity against the UNMODIFIED reference code: our GGUF parser, tokenizer and sampler (csrc/engine/{gguf,text}.cpp)
+against what the reference's GGUFLoader (src/model/loader.cpp:23-276), Tokenizer (src/inference/tokenizer.cpp:64-314) and Sampler
+(src/inference/sampler.cpp:18-117) returned on the same files and inputs, recorded in tests/golden/ref_host.json by
+tests/golden/make_ref_golden.py (oracle/_ref/libnt_ref.so, oracle/Makefile `ref`).  No GPU is involved: these are the host rows
+(a17, a18) of SURVEY §8, which the reference's own tests do not pin."""
 import ctypes as C
 import json
+from pathlib import Path
 
 import numpy as np
 import pytest
@@ -15,6 +16,14 @@ from ntransformer_b200.model_spec import TINY, LlamaConfig
 
 WORDS = ("the quick brown fox jumps over lazy dog hello world how are you today is a good day for inference tokens "
          "quantized decode tensor parallel kernel memory bandwidth roofline").split()
+
+
+GOLDEN = Path(__file__).resolve().parent / "golden" / "ref_host.json"
+
+
+@pytest.fixture(scope="module")
+def golden():
+    return json.loads(GOLDEN.read_text())
 
 
 def _setup(ref):
@@ -65,9 +74,7 @@ def spm_vocab(n):
     return toks[:n], types[:n]
 
 
-@pytest.fixture(scope="module")
-def files(tmp_path_factory):
-    d = tmp_path_factory.mktemp("refhost")
+def write_files(d):
     cfg = LlamaConfig(**{**TINY.dict(), "vocab_size": 1024})
     tensors = synthetic_tensors_np(cfg, "Q4_K_M", seed=3)
     rng = np.random.default_rng(0)
@@ -77,6 +84,11 @@ def files(tmp_path_factory):
     write_gguf(d / "spm.gguf", cfg, tensors, vocab_tokens=s, vocab_scores=rng.standard_normal(len(s)).astype(np.float32) - 5.0,
                vocab_types=types)
     return cfg, tensors, d / "gpt2.gguf", d / "spm.gguf"
+
+
+@pytest.fixture(scope="module")
+def files(tmp_path_factory):
+    return write_files(tmp_path_factory.mktemp("refhost"))
 
 
 TEXTS = ["Hello, how are you?", "hello world", " the quick  brown fox", "The Quick Brown Fox jumps over the lazy dog.", "", " ",
@@ -96,36 +108,48 @@ def ref_tokenize(ref, path, text, add_bos):
     return n, list(ids[: max(n, 0)])
 
 
+def random_id_lists(vocab_size):
+    """Arbitrary ids to decode: control / byte / placeholder tokens and out-of-range ids."""
+    rng = np.random.default_rng(1)
+    return [rng.integers(-2, vocab_size + 3, size=24).astype(np.int32) for _ in range(20)]
+
+
+def detokenize(fn, path, ids):
+    ids = np.ascontiguousarray(ids, dtype=np.int32)
+    out = C.create_string_buffer(8192)
+    n = fn(str(path).encode(), ids.ctypes.data_as(C.c_void_p), len(ids), out, 8192)
+    return [n, out.raw[:max(n, 0)].hex()]
+
+
+def record_tokenizer(ref, path, vocab_size):
+    """The reference's side of test_tokenizer_encode_decode_match_reference (tests/golden/make_ref_golden.py)."""
+    encode = [[list(ref_tokenize(ref, path, text, add_bos)) for add_bos in (True, False)] for text in TEXTS]
+    decode = [detokenize(ref.ref_detokenize, path, ids) if n > 0 else None for _, (n, ids) in encode]
+    return {"encode": encode, "decode": decode,
+            "decode_random": [detokenize(ref.ref_detokenize, path, ids) for ids in random_id_lists(vocab_size)]}
+
+
 @pytest.mark.parametrize("which", ["gpt2", "spm"])
-def test_tokenizer_encode_decode_match_reference(ref_lib, files, which, capfd):
-    ref = _setup(ref_lib)
+def test_tokenizer_encode_decode_match_reference(golden, files, which, capfd):
+    want = golden["tokenizer"][which]
     cfg, _, gpt2, spm = files
     path = gpt2 if which == "gpt2" else spm
-    for text in TEXTS:
-        for add_bos in (True, False):
-            a, b = ours_tokenize(path, text, add_bos), ref_tokenize(ref, path, text, add_bos)
-            assert a == b, (which, text, add_bos, a, b)
+    for text, enc, dec in zip(TEXTS, want["encode"], want["decode"]):
+        for add_bos, b in zip((True, False), enc):
+            a = ours_tokenize(path, text, add_bos)
+            assert list(a) == b, (which, text, add_bos, a, b)
         n, ids = ours_tokenize(path, text, False)
         if n == 0:
             continue
-        arr = (C.c_int * n)(*ids)
-        o1, o2 = C.create_string_buffer(8192), C.create_string_buffer(8192)
-        n1 = lib().nt_detokenize(str(path).encode(), arr, n, o1, 8192)
-        n2 = ref.ref_detokenize(str(path).encode(), arr, n, o2, 8192)
-        assert n1 == n2 and o1.raw[:n1] == o2.raw[:n2], (which, text)
+        assert detokenize(lib().nt_detokenize, path, ids) == dec, (which, text)
     # decoding arbitrary ids (control / byte / placeholder tokens, out-of-range ids) must agree too
-    rng = np.random.default_rng(1)
-    for _ in range(20):
-        ids = rng.integers(-2, cfg.vocab_size + 3, size=24).astype(np.int32)
-        o1, o2 = C.create_string_buffer(8192), C.create_string_buffer(8192)
-        n1 = lib().nt_detokenize(str(path).encode(), ids.ctypes.data_as(C.c_void_p), len(ids), o1, 8192)
-        n2 = ref.ref_detokenize(str(path).encode(), ids.ctypes.data_as(C.c_void_p), len(ids), o2, 8192)
-        assert n1 == n2 and o1.raw[:max(n1, 0)] == o2.raw[:max(n2, 0)], list(ids)
+    for ids, dec in zip(random_id_lists(cfg.vocab_size), want["decode_random"]):
+        assert detokenize(lib().nt_detokenize, path, ids) == dec, list(ids)
     capfd.readouterr()
 
 
-def test_sampler_draws_match_reference(ref_lib):
-    ref = _setup(ref_lib)
+def sampler_cases():
+    """Arguments of nt_sample_token / ref_sample_token: logits (with ties every 7th), settings and seed."""
     rng = np.random.default_rng(7)
     n = 2048
     for trial in range(60):
@@ -139,28 +163,47 @@ def test_sampler_draws_match_reference(ref_lib):
         window = int(rng.choice([0, 4, 64]))
         recent = rng.integers(0, n, size=int(rng.integers(0, 80))).astype(np.int32)
         seed = int(rng.integers(0, 2**31))
-        args = (logits.ctypes.data_as(C.c_void_p), n, temperature, top_k, top_p, penalty, window,
-                recent.ctypes.data_as(C.c_void_p) if len(recent) else None, len(recent), seed)
-        a = lib().nt_sample_token(*args)
-        b = ref.ref_sample_token(*args)
-        assert a == b, (trial, temperature, top_k, top_p, penalty, window, len(recent), seed, a, b)
+        yield (logits, n, temperature, top_k, top_p, penalty, window, recent, len(recent), seed)
 
 
-def test_gguf_parser_matches_reference_loader(ref_lib, files, capfd):
-    ref = _setup(ref_lib)
+def sample_args(case):
+    logits, n, temperature, top_k, top_p, penalty, window, recent, n_recent, seed = case
+    return (logits.ctypes.data_as(C.c_void_p), n, temperature, top_k, top_p, penalty, window,
+            recent.ctypes.data_as(C.c_void_p) if n_recent else None, n_recent, seed)
+
+
+def test_sampler_draws_match_reference(golden):
+    for trial, (case, b) in enumerate(zip(sampler_cases(), golden["sampler"], strict=True)):
+        a = lib().nt_sample_token(*sample_args(case))
+        assert a == b, (trial, case[2:7], case[8], case[9], a, b)
+
+
+def record_gguf(ref, path):
+    """The reference loader's view of the file (tests/golden/make_ref_golden.py)."""
+    buf = C.create_string_buffer(4 << 20)
+    assert lib().nt_gguf_describe(str(path).encode(), buf, len(buf)) > 0
+    out, fout = (C.c_longlong * 12)(), (C.c_float * 2)()
+    nt = ref.ref_gguf_config(str(path).encode(), out, fout)
+    tensors = {}
+    for t in json.loads(buf.value.decode())["tensors"]:
+        info = (C.c_longlong * 3)()
+        assert ref.ref_gguf_tensor(str(path).encode(), t["name"].encode(), info) == 0
+        tensors[t["name"]] = list(info)
+    return {"n_tensors": nt, "config": list(out), "norm_eps": fout[0], "rope_theta": fout[1], "tensors": tensors}
+
+
+def test_gguf_parser_matches_reference_loader(golden, files, capfd):
     cfg, tensors, gpt2, _ = files
+    want = golden["gguf"]
     buf = C.create_string_buffer(4 << 20)
     assert lib().nt_gguf_describe(str(gpt2).encode(), buf, len(buf)) > 0
     d = json.loads(buf.value.decode())
-    out, fout = (C.c_longlong * 12)(), (C.c_float * 2)()
-    nt = ref.ref_gguf_config(str(gpt2).encode(), out, fout)
-    assert nt == len(d["tensors"]) == len(tensors)
+    assert want["n_tensors"] == len(d["tensors"]) == len(tensors)
     keys = ("vocab_size", "hidden_size", "intermediate_size", "n_layers", "n_heads", "n_kv_heads", "head_dim", "max_seq_len",
             "bos_token_id", "eos_token_id", "n_vocab_tokens", "data_offset")
-    assert [d[k] for k in keys] == list(out)
-    assert abs(d["norm_eps"] - fout[0]) < 1e-12 and abs(d["rope_theta"] - fout[1]) < 1e-3
+    assert [d[k] for k in keys] == want["config"]
+    assert abs(d["norm_eps"] - want["norm_eps"]) < 1e-12 and abs(d["rope_theta"] - want["rope_theta"]) < 1e-3
+    assert len(want["tensors"]) == len(d["tensors"])
     for t in d["tensors"]:
-        info = (C.c_longlong * 3)()
-        assert ref.ref_gguf_tensor(str(gpt2).encode(), t["name"].encode(), info) == 0
-        assert (t["dtype"], t["offset"], t["nbytes"]) == tuple(info), t["name"]
+        assert [t["dtype"], t["offset"], t["nbytes"]] == want["tensors"][t["name"]], t["name"]
     capfd.readouterr()

@@ -1,7 +1,9 @@
 """The GPU sampler's kernel (csrc/sample.cu) executed on the CPU emulator (tests/cusim) against the UNMODIFIED reference
-sampler (oracle/_ref: src/inference/sampler.cpp) and our host sampler, on the same logits / settings / seed.  The kernel
-follows the reference's float operations in order, so draws must be identical whenever no ties straddle the top-k cut."""
+sampler (src/inference/sampler.cpp; its draws recorded in tests/golden/ref_host.json by tests/golden/make_ref_golden.py) and
+our host sampler, on the same logits / settings / seed.  The kernel follows the reference's float operations in order, so draws
+must be identical whenever no ties straddle the top-k cut."""
 import ctypes as C
+import json
 import subprocess
 from pathlib import Path
 
@@ -30,10 +32,9 @@ def args_for(logits, temperature, top_k, top_p, penalty, window, recent, seed):
             recent.ctypes.data_as(C.c_void_p) if len(recent) else None, len(recent), seed)
 
 
-def test_draws_match_the_reference_sampler(sim, ref_lib):
-    ref_lib.ref_sample_token.argtypes = SIG
+def draw_cases():
+    """Arguments of sample_sim / ref_sample_token / nt_sample_token (test_draws_match_the_reference_sampler)."""
     rng = np.random.default_rng(11)
-    checked = 0
     for trial in range(40):
         n = int(rng.choice([300, 2048, 5000, 33000]))
         logits = (rng.standard_normal(n) * rng.choice([0.5, 2.0, 6.0])).astype(np.float32)
@@ -46,11 +47,18 @@ def test_draws_match_the_reference_sampler(sim, ref_lib):
         if trial % 5 == 0 and len(recent) > 3:
             recent[-1] = recent[-2] = int(np.argmax(logits))             # the top token twice in the window: penalised twice
         seed = int(rng.integers(0, 2**31))
-        a = args_for(logits, temperature, top_k, top_p, penalty, window, recent, seed)
+        yield logits, temperature, top_k, top_p, penalty, window, recent, seed
+
+
+def test_draws_match_the_reference_sampler(sim):
+    wants = json.loads((ROOT / "tests" / "golden" / "ref_host.json").read_text())["sample_sim"]
+    checked = 0
+    for trial, (case, want) in enumerate(zip(draw_cases(), wants, strict=True)):
+        logits, temperature, top_k, top_p, penalty, window, recent, seed = case
+        a = args_for(*case)
         got = sim.sample_sim(*a)
-        want = ref_lib.ref_sample_token(*a)
         ours = lib().nt_sample_token(*a)
-        assert got == want == ours, (trial, n, temperature, top_k, top_p, penalty, window, seed, got, want, ours)
+        assert got == want == ours, (trial, len(logits), temperature, top_k, top_p, penalty, window, seed, got, want, ours)
         checked += 1
     assert checked == 40
 
